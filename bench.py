@@ -11,16 +11,20 @@ One step = one pass of the hot path over one batch.  `value` = device time (CUDA
 stream, inputs already in HBM); `e2e` = the same batch through the public C-ABI call with pinned HOST buffers,
 H2D + kernels + D2H of the verdicts inside the timed region.  `--impl reference` times the CPU restatement
 (oracle/, plain C; blst/ssz_rs themselves cannot be built offline — DESIGN.md) on the host cores.
+`--dump-outputs DIR` writes the verdict codes and the state root of the last timed step as DIR/<name>.npy.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import ctypes as C
 import hashlib
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
@@ -29,6 +33,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 
 R_ORDER = 0x73eda753299d7d483339d80809a1d80553bda402fffe5bfeffffffff00000001
 SEED = 0xB200
@@ -44,20 +49,23 @@ ORACLE_BUILD = "gcc -O3"   # set by load_oracles()
 
 # ------------------------------------------------------------------------------------------------ helpers
 def load_oracles():
-    import fcntl
-    with open(ROOT / "oracle" / ".build.lock", "w") as lk:  # ranks of one node must not rebuild the .so concurrently
-        fcntl.flock(lk, fcntl.LOCK_EX)
-        subprocess.run(["make", "-s", "-C", str(ROOT / "oracle")], check=True)
+    # the oracles build() compiled under oracle/; when they are missing or older than their sources, this process compiles
+    # its own copy into a temporary directory, since the tree may be read-only (and ranks then never share a build)
+    lib_dir = ROOT / "oracle"
+    if subprocess.run(["make", "-q", "-C", str(lib_dir)], capture_output=True).returncode != 0:
+        lib_dir = Path(tempfile.mkdtemp(prefix="b200_oracle_"))
+        atexit.register(shutil.rmtree, lib_dir, True)
+        subprocess.run(["make", "-s", "-C", str(ROOT / "oracle"), f"OUT={lib_dir}/"], check=True)
     # the timed CPU arm gets the mulx / adx build when this host's CPU has both features (same results, ~20 % faster products)
     global ORACLE_BUILD
     try:
         flags = set(next(ln for ln in open("/proc/cpuinfo") if ln.startswith("flags")).split())
     except (OSError, StopIteration):
         flags = set()
-    adx = {"adx", "bmi2"} <= flags and (ROOT / "oracle" / "liboracle_bls_adx.so").exists()
+    adx = {"adx", "bmi2"} <= flags and (lib_dir / "liboracle_bls_adx.so").exists()
     ORACLE_BUILD = "gcc -O3 -mbmi2 -madx" if adx else "gcc -O3"
-    bls = C.CDLL(str(ROOT / "oracle" / ("liboracle_bls_adx.so" if adx else "liboracle_bls.so")))
-    ssz = C.CDLL(str(ROOT / "oracle" / "liboracle_ssz.so"))
+    bls = C.CDLL(str(lib_dir / ("liboracle_bls_adx.so" if adx else "liboracle_bls.so")))
+    ssz = C.CDLL(str(lib_dir / "liboracle_ssz.so"))
     vp, sz, ci = C.c_void_p, C.c_size_t, C.c_int
     bls.orc_fast_aggregate_verify_batch.argtypes = [vp, vp, vp, vp, sz, vp, ci]
     bls.orc_sign_batch.argtypes = [vp, vp, sz, vp, ci]
@@ -161,6 +169,23 @@ def pin(arr):
     return t
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: what the timed paths returned in their last step, as DIR/<name>.npy in float64, so that two builds
+    run with the same arguments (hence the same seeded inputs) can be compared output for output.  An array larger than
+    its share of DUMP_BYTES is replaced by a fixed, seeded sample of its elements (same positions in every run)."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    cap = DUMP_BYTES // 8 // max(1, len(arrays))
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).ravel()
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(SEED).choice(a.size, cap, replace=False))]
+        np.save(d / f"{name}.npy", a)
+
+
 # ------------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -177,7 +202,10 @@ def main():
     ap.add_argument("--skip-rlc", action="store_true", help="skip the RLC whole-batch check")
     ap.add_argument("--skip-block", action="store_true", help="skip the configs[3] block signature set")
     ap.add_argument("--strong-tuples", type=int, default=2048)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write each timed path's last outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # Libraries (NCCL's version banner, make, ...) may write to fd 1; the contract is ONE JSON line on stdout from rank 0.
     real_stdout = os.dup(1)
     os.dup2(2, 1)
@@ -217,6 +245,8 @@ def main():
             if i >= args.warmup:
                 times.append(dt)
         assert out.tolist() == w["expect"].tolist(), "CPU restatement disagrees with the constructed verdicts"
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"fast_aggregate_verify_codes": out})
         ms = 1e3 * sum(times) / len(times)
         v = sample / (ms / 1e3)
         line = dict(base)
@@ -330,7 +360,7 @@ def main():
             sc = parallel.sharded_verify_batch(spk, soff, smsg, ssig)
         assert sc.tolist() == ws["expect"].tolist(), "sharded verdicts differ from the constructed expectation"
         s_wall, s_dev = [], []
-        for _ in range(max(3, args.steps)):
+        for _ in range(args.steps):
             flush_l2()
             barrier()
             t0 = time.perf_counter()
@@ -519,6 +549,9 @@ def main():
         })
     if strong is not None:
         line["epoch_batch_strong"] = strong
+    outputs = {"fast_aggregate_verify_codes": codes}
+    if strong is not None:
+        outputs["epoch_batch_codes"] = sc
 
     # ---------------------------------------------------------------- secondary: hash_tree_root(BeaconState)
     if not args.skip_ssz:
@@ -645,6 +678,7 @@ def main():
             resident_sharded = {"ms_wall_max_over_ranks": sum(r[0] for r in rs) / len(rs), "ms_device_max_over_ranks": sum(r[1] for r in rs) / len(rs)}
         if args.validators == 1 << 20 and golden:
             assert root.hex() == golden, "hash_tree_root(BeaconState) differs from the hashlib golden root"
+        outputs["beacon_state_root"] = np.frombuffer(root, dtype=np.uint8)
         if rank == 0:
             out32 = C.create_string_buffer(32)
             t0 = time.perf_counter()
@@ -685,6 +719,8 @@ def main():
                            "cpu_baseline": {"ms_1_thread": cpu1, f"ms_{host_threads}_threads": cpun, "kind": "port",
                                             "note": "plain-C restatement with SHA-NI when the host has it (not ssz_rs)"}}
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     parallel.comm_destroy()
     if world > 1:

@@ -1,5 +1,5 @@
-"""One rank of tests/test_config_scale_gpu.py::test_two_rank_sharded_calls_over_nccl (also runnable by hand under
-`gpurun --gpus 2`).  No torch: the library's communicator is created from a 128-byte id that rank 0 writes to a file —
+"""One rank of tests/test_config_scale_gpu.py::test_two_rank_sharded_calls_over_nccl (also runnable by hand on a
+machine with two GPUs).  No torch: the library's communicator is created from a 128-byte id that rank 0 writes to a file —
 the same bootstrap a Rust host would do over whatever channel it has."""
 import ctypes as C
 import json

@@ -165,7 +165,7 @@ def _gpu_count():
         return 0
 
 
-@pytest.mark.skipif(_gpu_count() < 2, reason="needs >= 2 GPUs on the box (gpurun --gpus 2)")
+@pytest.mark.skipif(_gpu_count() < 2, reason="needs >= 2 GPUs (one rank per GPU)")
 def test_two_rank_sharded_calls_over_nccl(tmp_path):
     """Two processes, one GPU each, NO torch: the library's own communicator (id handed over through a file), then the
     sharded state root and the sharded verify batch must agree with the single-GPU answers on both ranks."""
