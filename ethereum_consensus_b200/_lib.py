@@ -16,6 +16,7 @@ LIB_PATH = Path(os.environ.get("B200_LIB", PKG / "libb200_consensus.so"))  # B20
 SUCCESS, BAD_ENCODING, POINT_NOT_ON_CURVE, POINT_NOT_IN_GROUP = 0, 1, 2, 3
 AGGR_TYPE_MISMATCH, VERIFY_FAIL, PK_IS_INFINITY, BAD_SCALAR = 4, 5, 6, 7
 EMPTY_AGGREGATE = 16
+KZG_BAD_ARGS = 17
 ERR_CUDA, ERR_NO_DEVICE, ERR_BAD_ARG, ERR_SSZ_MALFORMED, ERR_NOT_INITIALIZED, ERR_LIMIT, ERR_COMM = 0x100, 0x101, 0x102, 0x103, 0x104, 0x105, 0x106
 PRESET = {"mainnet": 0, "minimal": 1}
 

@@ -198,6 +198,25 @@ template <class F> B200_BIG void jac_mul_u64(Jac<F>& r, const F& qx, const F& qy
     }
     r = acc;
 }
+// r = [k] * (qx, qy) for a 256-bit scalar given as 8 little-endian 32-bit limbs, left-to-right double-and-add over all
+// 256 bits (k = 0 gives infinity; doubling infinity keeps Z = 0).  The scalar is shifted out of the top limb, so it stays
+// in registers (no dynamically indexed limb array).
+template <class F> B200_BIG void jac_mul_u256(Jac<F>& r, const F& qx, const F& qy, const uint32_t k_in[8]) {
+    uint32_t k[8];
+#pragma unroll
+    for (int i = 0; i < 8; i++) k[i] = k_in[i];
+    Jac<F> acc;
+    jac_set_inf(acc);
+#pragma unroll 1
+    for (int bit = 0; bit < 256; bit++) {
+        jac_double(acc, acc);
+        if (k[7] >> 31) jac_add_mixed(acc, acc, qx, qy);
+#pragma unroll
+        for (int i = 7; i > 0; i--) k[i] = (k[i] << 1) | (k[i - 1] >> 31);
+        k[0] <<= 1;
+    }
+    r = acc;
+}
 // same for a Jacobian base point
 template <class F> B200_BIG void jac_mul_u64_jac(Jac<F>& r, const Jac<F>& q, uint64_t k) {
     Jac<F> acc;

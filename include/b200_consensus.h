@@ -42,6 +42,7 @@ enum {
     B200_PK_IS_INFINITY = 6,     /* BLST_PK_IS_INFINITY */
     B200_BAD_SCALAR = 7,         /* BLST_BAD_SCALAR */
     B200_EMPTY_AGGREGATE = 16,   /* Error::EmptyAggregate (crypto/bls.rs:80-82,136-138) */
+    B200_KZG_BAD_ARGS = 17,      /* kzg::Error::CKzg(..) (crypto/kzg.rs:47-53): malformed KZG input, see the KZG section */
     B200_ERR_CUDA = 0x100,
     B200_ERR_NO_DEVICE = 0x101,
     B200_ERR_BAD_ARG = 0x102,
@@ -256,6 +257,39 @@ B200_API int32_t b200_tune(const char* knob, int64_t value);
 B200_API int32_t b200_vm_load_programs(const uint32_t* blob, size_t n_words);
 /* On-device self-test of the field arithmetic over `n` pseudo-random triples; *mismatches must come back 0. */
 B200_API int32_t b200_fp_selftest(uint32_t n, uint32_t seed, uint32_t* mismatches);
+
+/* ---- KZG blob proofs, deneb (replaces the c_kzg verification calls of crypto/kzg.rs) ------------------------------- */
+/* Semantics of the deneb polynomial-commitments spec (what c-kzg implements).  Field elements (blob elements, z, y) are
+ * 32-byte big-endian integers that must be < r; commitments and proofs are 48-byte compressed G1 points that must
+ * decompress and lie in G1 (the infinity encoding is valid: the zero polynomial).  Results: 0 = Ok(()),
+ * B200_VERIFY_FAIL = Err(Error::InvalidProof), B200_KZG_BAD_ARGS = Err(Error::CKzg(..)) for any malformed input;
+ * engine failures stay >= 0x100.  A blob is 4 096 field elements = 131 072 bytes. */
+#define B200_KZG_BYTES_PER_BLOB 131072
+/* batch entry points take at most this many blobs per call (16 GiB of blobs would not fit the device anyway:
+ * each blob is 128 KiB of host-to-device copy) -> B200_ERR_BAD_ARG above it */
+#define B200_KZG_MAX_BLOBS 16384
+typedef struct b200_kzg_settings b200_kzg_settings;
+/* KzgSettings::load_trusted_setup — crypto/kzg.rs:39-45.  n_g1 must be 4 096 (g1_lagrange, natural order) and n_g2 >= 2
+ * (g2_monomial); every point must decode and lie in its subgroup, else B200_KZG_BAD_ARGS.  Only what verification uses
+ * stays resident: [tau]G2 = g2_monomial[1] and the bit-reversed roots of unity. */
+B200_API int32_t b200_kzg_settings_load(const uint8_t* g1_lagrange, size_t n_g1, const uint8_t* g2_monomial, size_t n_g2,
+                                        b200_kzg_settings** out);
+B200_API void b200_kzg_settings_free(b200_kzg_settings* settings);
+/* verify_kzg_proof — crypto/kzg.rs:101-122 */
+B200_API int32_t b200_verify_kzg_proof(const b200_kzg_settings* settings, const uint8_t commitment[48], const uint8_t z[32],
+                                       const uint8_t y[32], const uint8_t proof[48]);
+/* verify_blob_kzg_proof — crypto/kzg.rs:124-137 */
+B200_API int32_t b200_verify_blob_kzg_proof(const b200_kzg_settings* settings, const uint8_t* blob, const uint8_t commitment[48],
+                                            const uint8_t proof[48]);
+/* verify_blob_kzg_proof_batch — crypto/kzg.rs:139-174: one code for n blobs (n x 131 072, n x 48, n x 48 bytes).  n = 0
+ * returns 0; any malformed input returns B200_KZG_BAD_ARGS; otherwise 0 iff every blob's proof verifies.  The spec decides
+ * this with a random linear combination, which differs only with probability <= n / r; here every blob is checked. */
+B200_API int32_t b200_verify_blob_kzg_proof_batch(const b200_kzg_settings* settings, const uint8_t* blobs, const uint8_t* commitments,
+                                                  const uint8_t* proofs, size_t n);
+/* The throughput path (no counterpart in the reference): n independent blob checks in one call; out_codes[i] is exactly
+ * what b200_verify_blob_kzg_proof returns for blob i (which is this call with n = 1). */
+B200_API int32_t b200_verify_blob_kzg_proofs(const b200_kzg_settings* settings, const uint8_t* blobs, const uint8_t* commitments,
+                                             const uint8_t* proofs, size_t n, int32_t* out_codes);
 
 #ifdef __cplusplus
 }
