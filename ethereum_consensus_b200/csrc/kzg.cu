@@ -22,12 +22,8 @@
 #include "bls_kernels.cuh"
 #include "engine.h"
 #include "kzg_eval.cuh"
+#include "kzg_settings.h"
 #include "sha256.cuh"
-
-struct b200_kzg_settings {
-    b200::G2Aff* d_g2 = nullptr;   // [0] = -G2 (the generator, negated), [1] = [tau]G2 = g2_monomial[1]
-    b200::Fr* d_roots = nullptr;   // the 4 096 roots of unity in bit-reversed order, Montgomery form
-};
 
 namespace b200 {
 namespace {
@@ -359,6 +355,15 @@ int32_t kzg_run(Engine& e, KzgState& s, const b200_kzg_settings* st, KzgMode mod
 }
 
 }  // namespace
+
+// the prover (kzg_prove.cu) runs the challenge and the evaluation as they are
+void launch_kzg_challenge(const uint8_t* blobs, const uint8_t* comms, uint32_t n, Fr* z, cudaStream_t s) {
+    k_kzg_challenge<<<(n + 31) / 32, 32, 0, s>>>(blobs, comms, n, z);
+}
+void launch_kzg_eval(const uint8_t* blobs, const Fr* zs, const Fr* roots, Fr* ys, int32_t* codes, uint32_t n, cudaStream_t s) {
+    k_kzg_eval<<<n, kEvalThreads, 0, s>>>(blobs, zs, roots, ys, codes);
+}
+
 }  // namespace b200
 
 using namespace b200;
@@ -408,6 +413,7 @@ int32_t settings_load(Engine& e, const uint8_t* g1, size_t n_g1, const uint8_t* 
             if (codes[i] != BLS_SUCCESS && codes[i] != BLS_PK_IS_INFINITY) rc = B200_KZG_BAD_ARGS;
         for (size_t i = 0; i < n2 && !rc; i++)
             if (codes[n_g1 + i] != SIG_OK) rc = B200_KZG_BAD_ARGS;
+        if (!rc) rc = kzg_prover_settings_build(e, st, d_g1a, d_codes);   // the prover's bases, from the decoded points
     } while (0);
     cudaFree(d_g1b); cudaFree(d_g2b); cudaFree(d_g1a); cudaFree(d_g2a); cudaFree(d_codes);
     if (rc) { b200_kzg_settings_free(st); return rc; }
@@ -449,6 +455,8 @@ void b200_kzg_settings_free(b200_kzg_settings* st) {
     if (!st) return;
     cudaFree(st->d_g2);
     cudaFree(st->d_roots);
+    cudaFree(st->d_table);
+    cudaFree(st->d_base_inf);
     delete st;
 }
 

@@ -1,10 +1,11 @@
-"""Host-side mirror of `ethereum_consensus::crypto::kzg` (verification side), backed by the CUDA library — no CPU fallback.
+"""Host-side mirror of `ethereum_consensus::crypto::kzg`, backed by the CUDA library — no CPU fallback.
 
 Same names, argument order and errors as the reference's ethereum-consensus/src/crypto/kzg.rs: the byte-size constants
-(:5-9), `kzg_settings_from_json` (:39-45), `Error` with `CKzg` / `InvalidProof` (:47-53), `verify_kzg_proof` (:101-122),
-`verify_blob_kzg_proof` (:124-137) and `verify_blob_kzg_proof_batch` (:139-174).  `verify_blob_kzg_proofs` is the
-per-blob throughput path (one code per blob, no counterpart in the reference).  The prover side (`blob_to_kzg_commitment`,
-`compute_kzg_proof`, `compute_blob_kzg_proof`) is not implemented.
+(:5-9), `kzg_settings_from_json` (:39-45), `Error` with `CKzg` / `InvalidProof` (:47-53), `ProofAndEvaluation` (:55-59),
+`blob_to_kzg_commitment` (:60-69), `compute_kzg_proof` (:71-86), `compute_blob_kzg_proof` (:88-99), `verify_kzg_proof`
+(:101-122), `verify_blob_kzg_proof` (:124-137) and `verify_blob_kzg_proof_batch` (:139-174).  `verify_blob_kzg_proofs`,
+`blob_to_kzg_commitments` and `compute_blob_kzg_proofs` are the per-blob throughput paths (one code per blob, no
+counterpart in the reference).
 
 Rust `Result<(), Error>` becomes: return None on Ok, raise on Err.
 """
@@ -12,7 +13,8 @@ from __future__ import annotations
 
 import ctypes as C
 import json
-from typing import Sequence
+from dataclasses import dataclass
+from typing import Sequence, Tuple
 
 import numpy as np
 
@@ -34,6 +36,11 @@ _lib.register_protos({
     "b200_verify_blob_kzg_proof": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200_verify_blob_kzg_proof_batch": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "b200_verify_blob_kzg_proofs": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "b200_blob_to_kzg_commitment": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200_compute_kzg_proof": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200_compute_blob_kzg_proof": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200_blob_to_kzg_commitments": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "b200_compute_blob_kzg_proofs": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
 })
 
 
@@ -55,7 +62,8 @@ class InvalidProof(Error):
 
 
 class KzgSettings:
-    """Device-resident verification settings (`c_kzg::KzgSettings`): [tau]G2 and the bit-reversed roots of unity."""
+    """Device-resident settings (`c_kzg::KzgSettings`): [tau]G2 and the bit-reversed roots of unity for verification, and
+    the prover's fixed-base table built from g1_lagrange."""
 
     def __init__(self, g1_lagrange: bytes, g2_monomial: bytes):
         g1, g2 = bytes(g1_lagrange), bytes(g2_monomial)
@@ -170,3 +178,66 @@ def verify_blob_kzg_proofs(blobs, commitments, proofs, kzg_settings: KzgSettings
         _lib.check(_lib.init().b200_verify_blob_kzg_proofs(kzg_settings.handle, _lib.ptr(b), _lib.ptr(c), _lib.ptr(p), n,
                                                            out.ctypes.data), "b200_verify_blob_kzg_proofs")
     return out
+
+
+# ---------------------------------------------------------------------------------------------------- the prover
+@dataclass(frozen=True)
+class ProofAndEvaluation:
+    """crypto/kzg.rs:55-59: the proof and y = p(z), compared by value."""
+    proof: bytes
+    evaluation: bytes
+
+
+def blob_to_kzg_commitment(blob, kzg_settings: KzgSettings) -> bytes:
+    b = _bytes(blob, BYTES_PER_BLOB, "blob")
+    out = C.create_string_buffer(BYTES_PER_COMMITMENT)
+    _result(_lib.init().b200_blob_to_kzg_commitment(kzg_settings.handle, b, out), "b200_blob_to_kzg_commitment")
+    return out.raw
+
+
+def compute_kzg_proof(blob, evaluation_point, kzg_settings: KzgSettings) -> ProofAndEvaluation:
+    b = _bytes(blob, BYTES_PER_BLOB, "blob")
+    z = _bytes(evaluation_point, BYTES_PER_FIELD_ELEMENT, "evaluation point")
+    proof, y = C.create_string_buffer(BYTES_PER_PROOF), C.create_string_buffer(BYTES_PER_FIELD_ELEMENT)
+    _result(_lib.init().b200_compute_kzg_proof(kzg_settings.handle, b, z, proof, y), "b200_compute_kzg_proof")
+    return ProofAndEvaluation(proof.raw, y.raw)
+
+
+def compute_blob_kzg_proof(blob, commitment, kzg_settings: KzgSettings) -> bytes:
+    b = _bytes(blob, BYTES_PER_BLOB, "blob")
+    c = _bytes(commitment, BYTES_PER_COMMITMENT, "commitment")
+    out = C.create_string_buffer(BYTES_PER_PROOF)
+    _result(_lib.init().b200_compute_blob_kzg_proof(kzg_settings.handle, b, c, out), "b200_compute_blob_kzg_proof")
+    return out.raw
+
+
+def _check_count(n: int) -> None:
+    if n > MAX_BLOBS_PER_CALL:
+        raise ValueError(f"at most {MAX_BLOBS_PER_CALL} blobs per call, got {n}")
+
+
+def blob_to_kzg_commitments(blobs, kzg_settings: KzgSettings) -> Tuple[np.ndarray, np.ndarray]:
+    """(commitments uint8 [n, 48], codes int32 [n]): per blob 0 and its commitment, or 17 (an element >= r) and zeros.
+    `blobs` may be a sequence of bytes or a flat uint8 array (pinned tensors too)."""
+    b, n = _flat(blobs, BYTES_PER_BLOB, "blob")
+    _check_count(n)
+    out, codes = np.zeros((n, BYTES_PER_COMMITMENT), np.uint8), np.zeros(n, np.int32)
+    if n:
+        _lib.check(_lib.init().b200_blob_to_kzg_commitments(kzg_settings.handle, _lib.ptr(b), n, out.ctypes.data,
+                                                            codes.ctypes.data), "b200_blob_to_kzg_commitments")
+    return out, codes
+
+
+def compute_blob_kzg_proofs(blobs, commitments, kzg_settings: KzgSettings) -> Tuple[np.ndarray, np.ndarray]:
+    """(proofs uint8 [n, 48], codes int32 [n]): per blob what `compute_blob_kzg_proof` returns (0 and the proof, or 17
+    and zeros)."""
+    b, nb = _flat(blobs, BYTES_PER_BLOB, "blob")
+    c, nc = _flat(commitments, BYTES_PER_COMMITMENT, "commitment")
+    if nb != nc:
+        raise CKzgError(f"batch lengths differ: {nb} blobs, {nc} commitments")
+    _check_count(nb)
+    out, codes = np.zeros((nb, BYTES_PER_PROOF), np.uint8), np.zeros(nb, np.int32)
+    if nb:
+        _lib.check(_lib.init().b200_compute_blob_kzg_proofs(kzg_settings.handle, _lib.ptr(b), _lib.ptr(c), nb, out.ctypes.data,
+                                                            codes.ctypes.data), "b200_compute_blob_kzg_proofs")
+    return out, codes

@@ -270,8 +270,9 @@ B200_API int32_t b200_fp_selftest(uint32_t n, uint32_t seed, uint32_t* mismatche
 #define B200_KZG_MAX_BLOBS 16384
 typedef struct b200_kzg_settings b200_kzg_settings;
 /* KzgSettings::load_trusted_setup — crypto/kzg.rs:39-45.  n_g1 must be 4 096 (g1_lagrange, natural order) and n_g2 >= 2
- * (g2_monomial); every point must decode and lie in its subgroup, else B200_KZG_BAD_ARGS.  Only what verification uses
- * stays resident: [tau]G2 = g2_monomial[1] and the bit-reversed roots of unity. */
+ * (g2_monomial); every point must decode and lie in its subgroup, else B200_KZG_BAD_ARGS.  Resident on the device:
+ * [tau]G2 = g2_monomial[1] and the bit-reversed roots of unity (verification), and the prover's fixed-base table built
+ * from g1_lagrange in bit-reversed order (52 x 16 multiples of each point, 327 MB; built on the device at load time). */
 B200_API int32_t b200_kzg_settings_load(const uint8_t* g1_lagrange, size_t n_g1, const uint8_t* g2_monomial, size_t n_g2,
                                         b200_kzg_settings** out);
 B200_API void b200_kzg_settings_free(b200_kzg_settings* settings);
@@ -290,6 +291,25 @@ B200_API int32_t b200_verify_blob_kzg_proof_batch(const b200_kzg_settings* setti
  * what b200_verify_blob_kzg_proof returns for blob i (which is this call with n = 1). */
 B200_API int32_t b200_verify_blob_kzg_proofs(const b200_kzg_settings* settings, const uint8_t* blobs, const uint8_t* commitments,
                                              const uint8_t* proofs, size_t n, int32_t* out_codes);
+/* The prover.  Outputs are 48-byte compressed G1 points (the point at infinity is 0xc0 || 0^47) and, for
+ * compute_kzg_proof, y = p(z) as 32 big-endian bytes.  B200_KZG_BAD_ARGS: a blob element >= r, z >= r, or a commitment that
+ * does not decode or is not in G1 (infinity is valid); a failed call's outputs are zero.
+ * blob_to_kzg_commitment — crypto/kzg.rs:60-69 */
+B200_API int32_t b200_blob_to_kzg_commitment(const b200_kzg_settings* settings, const uint8_t* blob, uint8_t out_commitment[48]);
+/* compute_kzg_proof — crypto/kzg.rs:71-86: the proof of p(z) and y = p(z) (z on the domain takes the spec's in-domain branch) */
+B200_API int32_t b200_compute_kzg_proof(const b200_kzg_settings* settings, const uint8_t* blob, const uint8_t z[32],
+                                        uint8_t out_proof[48], uint8_t out_y[32]);
+/* compute_blob_kzg_proof — crypto/kzg.rs:88-99: the proof at z = compute_challenge(blob, commitment).  As in the spec, the
+ * commitment is not checked against the blob. */
+B200_API int32_t b200_compute_blob_kzg_proof(const b200_kzg_settings* settings, const uint8_t* blob, const uint8_t commitment[48],
+                                             uint8_t out_proof[48]);
+/* Throughput paths: n blobs in one call, one code per blob (what the single-blob call, which is this call with n = 1,
+ * returns); a failed blob's 48 output bytes are zero.  n = 0 returns 0 and writes nothing; n > B200_KZG_MAX_BLOBS returns
+ * B200_ERR_BAD_ARG.  Device scratch is bounded by the chunk of 1 024 blobs processed at a time (about 265 MiB). */
+B200_API int32_t b200_blob_to_kzg_commitments(const b200_kzg_settings* settings, const uint8_t* blobs, size_t n,
+                                              uint8_t* out_commitments, int32_t* out_codes);
+B200_API int32_t b200_compute_blob_kzg_proofs(const b200_kzg_settings* settings, const uint8_t* blobs, const uint8_t* commitments,
+                                              size_t n, uint8_t* out_proofs, int32_t* out_codes);
 
 #ifdef __cplusplus
 }
