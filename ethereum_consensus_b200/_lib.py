@@ -17,6 +17,7 @@ SUCCESS, BAD_ENCODING, POINT_NOT_ON_CURVE, POINT_NOT_IN_GROUP = 0, 1, 2, 3
 AGGR_TYPE_MISMATCH, VERIFY_FAIL, PK_IS_INFINITY, BAD_SCALAR = 4, 5, 6, 7
 EMPTY_AGGREGATE = 16
 KZG_BAD_ARGS = 17
+STATE_TRANSITION_INVALID = 18
 ERR_CUDA, ERR_NO_DEVICE, ERR_BAD_ARG, ERR_SSZ_MALFORMED, ERR_NOT_INITIALIZED, ERR_LIMIT, ERR_COMM = 0x100, 0x101, 0x102, 0x103, 0x104, 0x105, 0x106
 PRESET = {"mainnet": 0, "minimal": 1}
 
@@ -59,6 +60,10 @@ _PROTOS = {
     "b200_htr_beacon_state_deneb_combine": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
     "b200_compute_shuffled_indices": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint32, C.c_void_p]),
     "b200_get_active_validator_indices": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p, C.POINTER(C.c_size_t)]),
+    "b200_state_process_epoch_deneb": (C.c_int32, [C.c_void_p, C.c_uint32]),
+    "b200_state_process_slots_deneb": (C.c_int32, [C.c_void_p, C.c_uint64]),
+    "b200_state_serialized_len": (C.c_int32, [C.c_void_p, C.POINTER(C.c_size_t)]),
+    "b200_state_download_deneb": (C.c_int32, [C.c_void_p, C.c_void_p, C.c_size_t]),
     "b200_state_shuffled_active_indices": (C.c_int32, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p, C.POINTER(C.c_size_t)]),
     # multi-GPU (comm.cu): the exchange step lives inside the library
     "b200_comm_unique_id": (C.c_int32, [C.c_void_p]),

@@ -19,6 +19,7 @@
 #include "bls_kernels.cuh"
 #include "comm.h"
 #include "engine.h"
+#include "state_handle.h"
 
 namespace b200 {
 
@@ -948,15 +949,14 @@ int32_t b200_aggregate(const uint8_t* sigs_flat, size_t n, uint8_t out[96]) {
 }
 
 // crypto/bls.rs:135-148
-int32_t b200_eth_aggregate_public_keys(const uint8_t* pks_flat, size_t n, uint8_t out[48]) {
-    Engine& e = engine();
-    Guard g(e);
-    int32_t rc = check_ready(e);
-    if (rc) return rc;
+}  // extern "C"
+
+namespace b200 {
+int32_t eth_aggregate_public_keys_locked(Engine& e, const uint8_t* pks_flat, size_t n, uint8_t out[48]) {
     if (n == 0) return B200_EMPTY_AGGREGATE;
     if (!pks_flat || !out || n > 0x3fffffffu) return B200_ERR_BAD_ARG;
     BlsState* s;
-    rc = bls_state(e, &s);
+    int32_t rc = bls_state(e, &s);
     if (rc) return rc;
     B200_CUDA_TRY(s->keys.reserve(n * 48 + 64));
     B200_CUDA_TRY(s->key_aff.reserve((n + 1) * sizeof(G1Aff)));
@@ -987,6 +987,17 @@ int32_t b200_eth_aggregate_public_keys(const uint8_t* pks_flat, size_t n, uint8_
     const int32_t code = int32_t(h[4]);
     if (code == B200_SUCCESS) memcpy(out, h + 8, 48);
     return code;
+}
+}  // namespace b200
+
+extern "C" {
+
+int32_t b200_eth_aggregate_public_keys(const uint8_t* pks_flat, size_t n, uint8_t out[48]) {
+    Engine& e = engine();
+    Guard g(e);
+    int32_t rc = check_ready(e);
+    if (rc) return rc;
+    return eth_aggregate_public_keys_locked(e, pks_flat, n, out);
 }
 
 }  // extern "C"

@@ -10,6 +10,7 @@
 #include "sha256.cuh"
 #include "shuffle.h"
 #include "ssz_plan.h"
+#include "state_handle.h"
 
 namespace b200 {
 
@@ -65,41 +66,9 @@ int32_t run_oneshot(Engine& e, SszPlan& plan, const std::vector<uint32_t>& outpu
 
 using namespace b200;
 
-struct b200_state {
-    SszPlan plan;
-    std::vector<uint32_t> outputs;
-    DevBuf arena, fields, planbuf, selbuf, scatter;
-    bool uploaded = false;
-    // ---- incremental re-hash (b200_state_update_* / b200_state_root_incremental) ----
-    // Host shadow of the serialization with everything EXCEPT the five big lists filled in (their byte ranges stay
-    // untouched zero pages of an anonymous mapping): small-field updates patch it and the plan is rebuilt from it.
-    uint8_t* shadow = nullptr;
-    size_t len = 0;
-    int preset = 0;
-    StateOffsets so;
-    // per chain (5 big lists, then block_roots / state_roots / randao_mixes / slashings): changed first-job inputs
-    // (Validator records / 32-byte chunks), unsorted
-    std::vector<uint32_t> dirty[9];
-    bool small_dirty = false;
-    std::vector<std::pair<const uint8_t*, const uint8_t*>> small_ranges;  // patched shadow bytes since the last root
-    bool pinned_head = false, pinned_tail = false;
-    bool sharded = false;   // b200_state_upload_deneb_sharded: this rank's slices only; root is a collective, no updates
-    ~b200_state() {  // callers hold the engine lock and have selected the device
-        if (pinned_head) cudaHostUnregister(shadow);
-        if (pinned_tail) cudaHostUnregister(shadow + so.var[7]);
-        free(shadow);
-        arena.release(); fields.release(); planbuf.release(); selbuf.release(); scatter.release();
-    }
-};
-
 namespace {
-constexpr int kBigVar[5] = {2, 3, 4, 5, 6};         // StateOffsets::var index of each big list
-constexpr uint32_t kBigElem[5] = {121, 8, 1, 1, 8};  // element size in bytes
 // first-job input covering element i of big list f: a Validator record, or the 32-byte chunk of a packed list
 inline uint32_t big_input_of(int f, uint64_t i) { return uint32_t(f == 0 ? i : (i * kBigElem[f]) / 32); }
-inline uint64_t big_count(const b200_state* h, int f) {
-    return uint64_t(h->so.var[kBigVar[f] + 1] - h->so.var[kBigVar[f]]) / kBigElem[f];
-}
 }  // namespace
 
 extern "C" {
@@ -286,10 +255,7 @@ int32_t b200_state_upload_deneb(const uint8_t* ssz, size_t len, int32_t preset, 
     if (!h->shadow) { e.last_error = "out of host memory for the state shadow"; return B200_ERR_CUDA; }
     memcpy(h->shadow, ssz, h->so.var[2]);
     memcpy(h->shadow + h->so.var[7], ssz + h->so.var[7], len - h->so.var[7]);
-    // page-lock the two populated ranges (a few MB) so that re-staging a patched small field is a real async DMA
-    h->pinned_head = cudaHostRegister(h->shadow, h->so.var[2], cudaHostRegisterDefault) == cudaSuccess;
-    h->pinned_tail = cudaHostRegister(h->shadow + h->so.var[7], len - h->so.var[7], cudaHostRegisterDefault) == cudaSuccess;
-    cudaGetLastError();  // registration is an optimisation: pageable copies work too
+    h->pin();
     rc = build_beacon_state_plan(h->plan, h->shadow, len, preset, h->outputs);  // same layout: it depends on lengths only
     if (rc) return rc;
     h->uploaded = true;
@@ -312,23 +278,45 @@ static int32_t replan_if_small_dirty(Engine& e, b200_state* h) {
     return B200_SUCCESS;
 }
 
+}  // extern "C"
+
+namespace b200 {
+int32_t state_root_locked(Engine& e, b200_state* h, bool incremental, uint8_t out[32]) {
+    int32_t rc = replan_if_small_dirty(e, h);  // updates made through b200_state_update_* are honoured here too
+    if (rc) return rc;
+    const CopyMode copy = (h->small_dirty || h->relaid) ? COPY_SMALL_ONLY : COPY_NONE;
+    // after a re-layout every small field is re-staged (no range filter)
+    const auto* ranges = h->relaid ? nullptr : &h->small_ranges;
+    if (incremental && !h->all_dirty && !h->relaid) {
+        std::vector<std::vector<uint32_t>> dirty(h->plan.n_chains());
+        for (int f = 0; f < 9 && size_t(f) < dirty.size(); f++) {
+            dirty[size_t(f)] = h->dirty[f];
+            std::sort(dirty[size_t(f)].begin(), dirty[size_t(f)].end());
+            dirty[size_t(f)].erase(std::unique(dirty[size_t(f)].begin(), dirty[size_t(f)].end()), dirty[size_t(f)].end());
+        }
+        rc = h->plan.run(e, h->arena, h->fields, h->planbuf, copy, h->outputs, out, &dirty, &h->selbuf, ranges);
+    } else {
+        rc = h->plan.run(e, h->arena, h->fields, h->planbuf, copy, h->outputs, out, nullptr, nullptr, ranges);
+    }
+    if (rc) return rc;
+    for (auto& d : h->dirty) d.clear();  // a full re-hash covers every dirty path
+    h->small_dirty = h->all_dirty = h->relaid = false;
+    h->small_ranges.clear();
+    return B200_SUCCESS;
+}
+}  // namespace b200
+
+extern "C" {
+
 int32_t b200_state_root(b200_state* h, uint8_t out[32]) {
     Engine& e = engine();
     Guard g(e);
     int32_t rc = check_ready(e);
     if (rc) return rc;
-    if (!h || !h->uploaded || !out) return B200_ERR_BAD_ARG;
+    if (!h || !h->uploaded || h->failed || !out) return B200_ERR_BAD_ARG;
     if (h->sharded)   // every rank of the communicator calls this together: stages | ncclAllGather | finisher
         return h->plan.run(e, h->arena, h->fields, h->planbuf, COPY_NONE, h->outputs, out);
-    rc = replan_if_small_dirty(e, h);  // updates made through b200_state_update_* are honoured here too
-    if (rc) return rc;
-    rc = h->plan.run(e, h->arena, h->fields, h->planbuf, h->small_dirty ? COPY_SMALL_ONLY : COPY_NONE, h->outputs, out,
-                     nullptr, nullptr, &h->small_ranges);
-    if (rc) return rc;
-    for (auto& d : h->dirty) d.clear();  // a full re-hash covers every dirty path
-    h->small_dirty = false;
-    h->small_ranges.clear();
-    return B200_SUCCESS;
+    return state_root_locked(e, h, false, out);
 }
 
 void b200_state_free(b200_state* h) {
@@ -344,7 +332,7 @@ int32_t b200_state_update_elements(b200_state* h, int32_t field, const uint64_t*
     Guard g(e);
     int32_t rc = check_ready(e);
     if (rc) return rc;
-    if (!h || !h->uploaded || h->sharded || field < 0 || field > 4 || (n && (!indices || !values)) || n > 0xffffffffull) return B200_ERR_BAD_ARG;
+    if (!h || !h->uploaded || h->failed || h->sharded || field < 0 || field > 4 || (n && (!indices || !values)) || n > 0xffffffffull) return B200_ERR_BAD_ARG;
     if (!n) return B200_SUCCESS;
     const uint64_t count = big_count(h, field);
     for (size_t i = 0; i < n; i++)
@@ -374,8 +362,15 @@ int32_t b200_state_update_bytes(b200_state* h, uint64_t ssz_offset, const uint8_
     Guard g(e);
     int32_t rc = check_ready(e);
     if (rc) return rc;
-    if (!h || !h->uploaded || h->sharded || (n && !data) || ssz_offset > h->len || n > h->len - ssz_offset) return B200_ERR_BAD_ARG;
+    if (!h || !h->uploaded || h->failed || h->sharded || (n && !data) || ssz_offset > h->len || n > h->len - ssz_offset) return B200_ERR_BAD_ARG;
     if (!n) return B200_SUCCESS;
+    return state_patch_bytes(e, h, ssz_offset, data, n);
+}
+
+}  // extern "C"
+
+namespace b200 {
+int32_t state_patch_bytes(Engine& e, b200_state* h, uint64_t ssz_offset, const uint8_t* data, size_t n) {
     const uint64_t lo = ssz_offset, hi = ssz_offset + n;
     // (1) the parts outside the big lists: patch the shadow; the variable-size offsets must not change
     std::vector<uint8_t> saved;
@@ -431,26 +426,125 @@ int32_t b200_state_update_bytes(b200_state* h, uint64_t ssz_offset, const uint8_
     return B200_SUCCESS;
 }
 
+// Variable-size offsets live in the fixed part: the position of each one (StateOffsets::var order, var[9] = end excluded)
+static void var_offset_positions(const StateOffsets& so, size_t sc_bytes, size_t pos[9]) {
+    pos[0] = so.eth1_data - 4;
+    pos[1] = so.eth1_deposit_index - 4;
+    pos[2] = so.eth1_deposit_index + 8;
+    pos[3] = pos[2] + 4;
+    pos[4] = so.justification_bits - 8;
+    pos[5] = so.justification_bits - 4;
+    pos[6] = so.checkpoints + 120;
+    pos[7] = so.next_sync_committee + sc_bytes;
+    pos[8] = so.next_withdrawal_validator_index + 8;
+}
+
+int32_t state_relayout(Engine& e, b200_state* h, int var, const uint8_t* bytes, size_t n) {
+    if (var < 0 || var > 8 || (var >= 2 && var <= 6)) return B200_ERR_BAD_ARG;   // never a big list
+    const StateOffsets old = h->so;
+    const size_t old_n = size_t(old.var[var + 1] - old.var[var]);
+    const size_t new_len = h->len - old_n + n;
+    if (new_len > 0xffffffffull) return B200_ERR_BAD_ARG;
+    uint8_t* ns = static_cast<uint8_t*>(calloc(new_len ? new_len : 1, 1));
+    if (!ns) { e.last_error = "out of host memory for the state shadow"; return B200_ERR_CUDA; }
+    // head and tail without the big lists (their ranges stay zero pages), with `var` replaced
+    auto copy_shifted = [&](size_t a, size_t b) {  // old range [a, b) that lies entirely before or after `var`
+        const size_t shift = a >= old.var[var + 1] ? (n - old_n) : 0;
+        memcpy(ns + a + shift, h->shadow + a, b - a);
+    };
+    if (var < 2) {
+        copy_shifted(0, old.var[var]);
+        memcpy(ns + old.var[var], bytes, n);
+        copy_shifted(old.var[var + 1], old.var[2]);
+        copy_shifted(old.var[7], h->len);
+    } else {
+        copy_shifted(0, old.var[2]);
+        copy_shifted(old.var[7], old.var[var]);
+        memcpy(ns + old.var[var], bytes, n);
+        copy_shifted(old.var[var + 1], h->len);
+    }
+    size_t pos[9];
+    const size_t sc_bytes = old.current_sync_committee < old.next_sync_committee ? old.next_sync_committee - old.current_sync_committee : 0;
+    var_offset_positions(old, sc_bytes, pos);
+    for (int i = var + 1; i < 9; i++) {
+        const uint32_t v = uint32_t(old.var[i] + n - old_n);
+        for (int k = 0; k < 4; k++) ns[pos[i] + k] = uint8_t(v >> (8 * k));
+    }
+    StateOffsets so2;
+    if (!parse_beacon_state(ns, new_len, h->preset, so2)) { free(ns); e.last_error = "re-layout: malformed result"; return B200_ERR_BAD_ARG; }
+    SszPlan np;
+    std::vector<uint32_t> outs;
+    int32_t rc = build_beacon_state_plan(np, ns, new_len, h->preset, outs);
+    if (rc || np.n_chains() != h->plan.n_chains()) { free(ns); return rc ? rc : B200_ERR_BAD_ARG; }
+    // fresh field buffer; every chain (big lists and big vectors) moves device to device, padding included
+    DevBuf nf;
+    cudaError_t ce = nf.reserve(np.field_bytes() + 256);
+    if (ce != cudaSuccess) { free(ns); e.last_error = cudaGetErrorString(ce); return B200_ERR_CUDA; }
+    for (int c = 0; c < int(np.n_chains()); c++) {
+        uint64_t fo = 0, fn = 0; size_t nb = 0, nb2 = 0;
+        const bool a = h->plan.chain_field(c, &fo, &nb), b = np.chain_field(c, &fn, &nb2);
+        if (a != b || nb != nb2) { nf.release(); free(ns); e.last_error = "re-layout: chain size changed"; return B200_ERR_BAD_ARG; }
+        if (!a || !nb) continue;
+        const size_t padded = (nb + 255) & ~size_t(255);
+        ce = cudaMemcpyAsync(static_cast<uint8_t*>(nf.p) + fn, static_cast<const uint8_t*>(h->fields.p) + fo, padded,
+                             cudaMemcpyDeviceToDevice, e.stream);
+        if (ce != cudaSuccess) { nf.release(); free(ns); e.last_error = cudaGetErrorString(ce); return B200_ERR_CUDA; }
+    }
+    ce = cudaStreamSynchronize(e.stream);
+    if (ce != cudaSuccess) { nf.release(); free(ns); e.last_error = cudaGetErrorString(ce); return B200_ERR_CUDA; }
+    h->unpin();
+    free(h->shadow);
+    h->fields.release();
+    h->fields = nf;
+    h->shadow = ns; h->len = new_len; h->so = so2;
+    h->plan = std::move(np); h->outputs = std::move(outs);
+    h->pin();
+    h->relaid = true;
+    h->small_dirty = false;
+    h->small_ranges.clear();
+    return B200_SUCCESS;
+}
+}  // namespace b200
+
+extern "C" {
+
 int32_t b200_state_root_incremental(b200_state* h, uint8_t out[32]) {
     Engine& e = engine();
     Guard g(e);
     int32_t rc = check_ready(e);
     if (rc) return rc;
-    if (!h || !h->uploaded || !out) return B200_ERR_BAD_ARG;
-    rc = replan_if_small_dirty(e, h);
+    if (!h || !h->uploaded || h->failed || h->sharded || !out) return B200_ERR_BAD_ARG;
+    return state_root_locked(e, h, true, out);
+}
+
+int32_t b200_state_serialized_len(b200_state* h, size_t* out_len) {
+    Engine& e = engine();
+    Guard g(e);
+    int32_t rc = check_ready(e);
     if (rc) return rc;
-    std::vector<std::vector<uint32_t>> dirty(h->plan.n_chains());
-    for (int f = 0; f < 9 && size_t(f) < dirty.size(); f++) {
-        dirty[size_t(f)] = h->dirty[f];
-        std::sort(dirty[size_t(f)].begin(), dirty[size_t(f)].end());
-        dirty[size_t(f)].erase(std::unique(dirty[size_t(f)].begin(), dirty[size_t(f)].end()), dirty[size_t(f)].end());
+    if (!h || !h->uploaded || h->failed || h->sharded || !out_len) return B200_ERR_BAD_ARG;
+    *out_len = h->len;
+    return B200_SUCCESS;
+}
+
+// The shadow with the five big lists copied back from HBM
+int32_t b200_state_download_deneb(b200_state* h, uint8_t* out, size_t cap) {
+    Engine& e = engine();
+    Guard g(e);
+    int32_t rc = check_ready(e);
+    if (rc) return rc;
+    if (!h || !h->uploaded || h->failed || h->sharded || !out || cap < h->len) return B200_ERR_BAD_ARG;
+    memcpy(out, h->shadow, h->so.var[2]);
+    memcpy(out + h->so.var[7], h->shadow + h->so.var[7], h->len - h->so.var[7]);
+    for (int f = 0; f < 5; f++) {
+        const size_t nb = size_t(h->so.var[kBigVar[f] + 1] - h->so.var[kBigVar[f]]);
+        if (!nb) continue;
+        uint64_t field_off = 0; size_t staged = 0;
+        if (!h->plan.chain_field(f, &field_off, &staged) || staged != nb) return B200_ERR_BAD_ARG;
+        B200_CUDA_TRY(cudaMemcpyAsync(out + h->so.var[kBigVar[f]], static_cast<const uint8_t*>(h->fields.p) + field_off, nb,
+                                      cudaMemcpyDeviceToHost, e.stream));
     }
-    rc = h->plan.run(e, h->arena, h->fields, h->planbuf, h->small_dirty ? COPY_SMALL_ONLY : COPY_NONE, h->outputs, out,
-                     &dirty, &h->selbuf, &h->small_ranges);
-    if (rc) return rc;
-    for (auto& d : h->dirty) d.clear();
-    h->small_dirty = false;
-    h->small_ranges.clear();
+    B200_CUDA_TRY(cudaStreamSynchronize(e.stream));
     return B200_SUCCESS;
 }
 
@@ -490,7 +584,7 @@ int32_t b200_state_shuffled_active_indices(b200_state* h, uint64_t epoch, const 
     Guard g(e);
     int32_t rc = check_ready(e);
     if (rc) return rc;
-    if (!h || !h->uploaded || h->sharded || !seed || !out_n) return B200_ERR_BAD_ARG;
+    if (!h || !h->uploaded || h->failed || h->sharded || !seed || !out_n) return B200_ERR_BAD_ARG;
     *out_n = 0;
     const uint64_t n = big_count(h, 0);
     if (n == 0) return B200_SUCCESS;

@@ -152,6 +152,14 @@ class DeviceBeaconState:
         _rc(_lib.lib().b200_state_root_incremental(self._h, out), "state_root_incremental")
         return bytes(out)
 
+    def to_ssz(self) -> np.ndarray:
+        """SSZ serialization of the current resident state (the big lists come back from HBM)."""
+        n = C.c_size_t(0)
+        _rc(_lib.lib().b200_state_serialized_len(self._h, C.byref(n)), "state_serialized_len")
+        out = np.empty(n.value, dtype=np.uint8)
+        _rc(_lib.lib().b200_state_download_deneb(self._h, _lib.ptr(out), out.size), "state_download")
+        return out
+
     def close(self) -> None:
         if self._h:
             _lib.lib().b200_state_free(self._h)

@@ -43,6 +43,7 @@ enum {
     B200_BAD_SCALAR = 7,         /* BLST_BAD_SCALAR */
     B200_EMPTY_AGGREGATE = 16,   /* Error::EmptyAggregate (crypto/bls.rs:80-82,136-138) */
     B200_KZG_BAD_ARGS = 17,      /* kzg::Error::CKzg(..) (crypto/kzg.rs:47-53): malformed KZG input, see the KZG section */
+    B200_STATE_TRANSITION_INVALID = 18, /* epoch / slot processing: a uint64 overflow or a failed spec assertion */
     B200_ERR_CUDA = 0x100,
     B200_ERR_NO_DEVICE = 0x101,
     B200_ERR_BAD_ARG = 0x102,
@@ -138,6 +139,39 @@ B200_API int32_t b200_get_active_validator_indices(const uint8_t* validators_ssz
  * [len*index/count, len*(index+1)/count) of `out` (compute_committee, :459-483). */
 B200_API int32_t b200_state_shuffled_active_indices(b200_state* handle, uint64_t epoch, const uint8_t seed[32], uint32_t rounds,
                                                     uint64_t* out, size_t* out_n);
+
+/* ---- epoch and slot processing on a device-resident state (deneb/spec/mod.rs:965-1004, :3150-3240) ---------------
+ * b200_state_process_epoch_deneb runs the process_epoch stages whose bits are set in `stage_mask`, in this order:
+ *   0 justification_and_finalization, 1 inactivity_updates, 2 rewards_and_penalties, 3 registry_updates, 4 slashings,
+ *   5 eth1_data_reset, 6 effective_balance_updates, 7 slashings_reset, 8 randao_mixes_reset,
+ *   9 historical_summaries_update, 10 participation_flag_updates, 11 sync_committee_updates.
+ * B200_EPOCH_ALL is process_epoch; a single bit is one epoch_processing sub-function.  The state stays in HBM: the
+ * next b200_state_root / b200_state_root_incremental returns the post-state root.
+ * b200_state_process_slots_deneb follows process_slots up to `slot` (process_epoch at each epoch boundary);
+ * slot <= state.slot returns B200_ERR_BAD_ARG (TransitionToPreviousSlot).
+ * Codes: B200_STATE_TRANSITION_INVALID for a uint64 overflow (the spec's rule; the reference Rust wraps or panics) or
+ * a failed spec assertion; 1..7 for an invalid public key in the next sync committee (as b200_eth_aggregate_public_keys).
+ * After either, the handle is failed: every later call on it returns B200_ERR_BAD_ARG until it is freed.  Sharded
+ * handles, an empty registry and lists whose lengths differ from the registry's return B200_ERR_BAD_ARG. */
+#define B200_EPOCH_JUSTIFICATION_AND_FINALIZATION (1u << 0)
+#define B200_EPOCH_INACTIVITY_UPDATES (1u << 1)
+#define B200_EPOCH_REWARDS_AND_PENALTIES (1u << 2)
+#define B200_EPOCH_REGISTRY_UPDATES (1u << 3)
+#define B200_EPOCH_SLASHINGS (1u << 4)
+#define B200_EPOCH_ETH1_DATA_RESET (1u << 5)
+#define B200_EPOCH_EFFECTIVE_BALANCE_UPDATES (1u << 6)
+#define B200_EPOCH_SLASHINGS_RESET (1u << 7)
+#define B200_EPOCH_RANDAO_MIXES_RESET (1u << 8)
+#define B200_EPOCH_HISTORICAL_SUMMARIES_UPDATE (1u << 9)
+#define B200_EPOCH_PARTICIPATION_FLAG_UPDATES (1u << 10)
+#define B200_EPOCH_SYNC_COMMITTEE_UPDATES (1u << 11)
+#define B200_EPOCH_ALL 0xfffu
+B200_API int32_t b200_state_process_epoch_deneb(b200_state* handle, uint32_t stage_mask);
+B200_API int32_t b200_state_process_slots_deneb(b200_state* handle, uint64_t slot);
+/* SSZ serialization of the current resident state (small fields from the host shadow, the five big lists copied back
+ * from HBM).  `cap` must be at least b200_state_serialized_len. */
+B200_API int32_t b200_state_serialized_len(b200_state* handle, size_t* out_len);
+B200_API int32_t b200_state_download_deneb(b200_state* handle, uint8_t* out, size_t cap);
 
 /* ---- multi-GPU: one process per GPU, the exchange step lives INSIDE the library (SURVEY.md §8b `b200_init(n_gpus)`,
  * §8e).  The reference is single-process (no counterpart, SURVEY.md §2a); a Rust host with one process per GPU calls:
